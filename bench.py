@@ -8,7 +8,8 @@ One "step" = one pass of the whole hot path over one batch of synthetic 150-bp p
 Timing: CUDA events on the library's own stream (elp_timer_start/stop), barrier + synchronize on both sides, max over ranks.
 Each step re-ingests ~270 B/read (>> the 126 MB L2), so no kernel ever sees a warm L2 from the previous step.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--reads R] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--reads R] [--impl reference] [--dump-outputs DIR]
+--dump-outputs DIR writes what the last timed step returned to its caller as DIR/<name>.npy (float32/float64, < 64 MB; see dump_outputs).
 N>1 is launched by torchrun (one rank per GPU): ONE hg38-shaped genome is partitioned over the ranks by contig group (sfm-style,
 cmd/sfm.go); 1 % of the pairs span two groups.  All cross-GPU traffic of the hot path is NCCL inside the library (C ABI): the spread-pair
 exchange of elp_sort_markdup (grouped ncclSend/ncclRecv of 128-byte mate records) and one ncclAllReduce of the integer BQSR tables.  --impl reference times the CPU restatement of the reference algorithm (oracle/, the Go
@@ -29,10 +30,13 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark leaves the source tree as it found it (it may be read-only)
 
 METRIC = "reads/sec through sort+markdup+BQSR"
 DEFAULT_READS = 30_000_000          # configs[1] scale (WES-scale 30M reads), with the full sort+markdup+BQSR path of configs[2]
 GENOME_SCALE = 20.0                 # hg38 / 20 = 155 Mbp  ->  30 M x 150 bp = 29x coverage, WGS-30x-like group statistics
+DUMP_ROWS = 1 << 16                 # --dump-outputs: output records in the seeded sample (all of them below this)
+DUMP_QUAL_MAX = 10_000_000          # --dump-outputs: QUAL bytes at most (40 MB as float32)
 
 
 def log(*a):
@@ -147,6 +151,25 @@ def verify_against_oracle(ctx, w, out_np, n_reads, threads):
             "against": "oracle/ (C restatement of the reference) on the same reads", "seconds": round(time.time() - t0, 1)}
 
 
+def dump_outputs(path, out_np, n_reads, tables, emp, suffix=""):
+    """what a caller of the timed path receives after a step, as path/<name><suffix>.npy for output-by-output comparison of two builds:
+    the BQSR table counters and EmpiricalQuality in full, and for a fixed seeded sample of output positions (every position when there
+    are at most DUMP_ROWS) the input record index, FLAG and QUAL there.  qual holds the QUAL bytes of the sampled records back to back
+    (qual_len of each), cut at DUMP_QUAL_MAX bytes; integers are exact in the float type they are stored as."""
+    idx, flag, qoff, qual = out_np
+    rows = np.arange(n_reads) if n_reads <= DUMP_ROWS else np.unique(np.random.default_rng(20260924).integers(0, n_reads, DUMP_ROWS))
+    lo, hi = qoff[rows].astype(np.int64), qoff[rows + 1].astype(np.int64)
+    keep = np.cumsum(hi - lo) <= DUMP_QUAL_MAX
+    rows, lo, lens = rows[keep], lo[keep], (hi - lo)[keep]
+    at = np.repeat(lo - (np.cumsum(lens) - lens), lens) + np.arange(int(lens.sum()))
+    arrays = {"rows": rows.astype(np.float64), "order": idx[rows].astype(np.float64), "flag": flag[rows].astype(np.float32),
+              "qual_len": lens.astype(np.float32), "qual": qual[at].astype(np.float32),
+              "bqsr_tables": np.asarray(tables).astype(np.float64), "empirical_quality": np.asarray(emp).astype(np.float32)}
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, f"{name}{suffix}.npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -159,7 +182,12 @@ def main():
     ap.add_argument("--e2e-contexts", type=int, default=3, choices=(1, 3), help="contexts in the e2e pipeline ring (1: sequential, for runs where one context fills the HBM)")
     ap.add_argument("--verify", dest="verify", action="store_true", default=None, help="check the last step's output against the oracle (default: on at --gpus 1)")
     ap.add_argument("--no-verify", dest="verify", action="store_false")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     rank, world, local = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1)), int(os.environ.get("LOCAL_RANK", 0))
     from elprep_b200 import synth
     all_contigs = synth.scaled_hg38(GENOME_SCALE / world)     # weak scaling: the genome grows with the number of GPUs, ~155 Mbp (29x coverage) per contig group
@@ -286,6 +314,8 @@ def main():
         dev_ms.append(a); in_ms.append(b); out_ms.append(c_); coll_ms.append(d_)
     launches = ctx.launch_count()
     stats = ctx.kernel_stats()
+    if args.dump_outputs:           # untimed, before the e2e run below reuses the context and the output buffers
+        dump_outputs(args.dump_outputs, out_np, n_reads, ctx.tables_get(), ctx.empirical_get(), f"_rank{rank}" if world > 1 else "")
     # ---- e2e: the same K steps through the public API with host buffers, software-pipelined over a ring of three contexts: while the
     # batch of step s uploads into one context, the context of step s-1 runs its device phases and starts its download, and the download of
     # step s-2 drains into the other of two page-locked output buffers.  The host->device copy engine -- the longest stage -- never waits.

@@ -93,8 +93,8 @@ class FakeEvent:
     def elapsed_time(self, other): return 1e3 * (other.t - self.t)
 
 
-@pytest.mark.parametrize("extra", [[], ["--e2e-contexts", "1", "--steps", "1"]])
-def test_bench_main_runs_and_prints_one_contract_line(monkeypatch, extra):
+def _fake_gpu_bench(monkeypatch):
+    """bench.py with the fake device, its torch.cuda calls stubbed and a ~1 Mbp genome"""
     import torch
     sys.path.insert(0, ROOT)
     import bench
@@ -113,14 +113,23 @@ def test_bench_main_runs_and_prints_one_contract_line(monkeypatch, extra):
     monkeypatch.setattr(bench, "GENOME_SCALE", 3000.0)              # a ~1 Mbp genome for 12 k reads
     for k in ("RANK", "WORLD_SIZE", "LOCAL_RANK"):
         monkeypatch.delenv(k, raising=False)
-    argv = ["bench.py", "--reads", "12000", "--steps", "4", "--warmup", "1", "--cpu-sample", "6000"] + extra
-    monkeypatch.setattr(sys, "argv", argv)
+    return bench
+
+
+def _run_bench(monkeypatch, bench, argv):
+    monkeypatch.setattr(sys, "argv", ["bench.py"] + argv)
     buf = io.StringIO()
     with redirect_stdout(buf):
         bench.main()
     lines = [ln for ln in buf.getvalue().splitlines() if ln.strip()]
     assert len(lines) == 1, lines                                   # exactly one JSON line on stdout
-    d = json.loads(lines[0])
+    return json.loads(lines[0])
+
+
+@pytest.mark.parametrize("extra", [[], ["--e2e-contexts", "1", "--steps", "1"]])
+def test_bench_main_runs_and_prints_one_contract_line(monkeypatch, extra):
+    bench = _fake_gpu_bench(monkeypatch)
+    d = _run_bench(monkeypatch, bench, ["--reads", "12000", "--steps", "4", "--warmup", "1", "--cpu-sample", "6000"] + extra)
     for key in ("metric", "value", "unit", "n_gpus", "steps", "warmup", "ms_per_step", "higher_is_better", "scaling", "vs_baseline", "dtype", "data", "config",
                 "e2e", "roofline", "roofline_graded", "cpu_baseline", "clocks", "gpu_launches", "verified"):
         assert key in d, key
@@ -131,6 +140,40 @@ def test_bench_main_runs_and_prints_one_contract_line(monkeypatch, extra):
     assert (e["steady_ms_per_step"] is None) == bool(extra)         # needs >= 3 pipelined steps
     assert d["roofline"]["kernel"] == "bqsr_apply" and 0 < d["roofline"]["frac"] and set(d["roofline_graded"]) == {"radix_sort", "covariate_histogram"}
     assert d["cpu_baseline"]["kind"] == "port" and d["cpu_baseline"]["value"] > 0 and d["gpu_launches"] > 0
+
+
+def test_bench_steps_and_dump_outputs(monkeypatch, tmp_path):
+    """--steps is the number of timed steps (the fake launches 49 kernels a step); --dump-outputs writes, as float arrays under 64 MB, the
+    outputs the last timed step fetched (a seeded sample of output positions, QUAL cut at DUMP_QUAL_MAX bytes), the same on every run"""
+    bench = _fake_gpu_bench(monkeypatch)
+    monkeypatch.setattr(bench, "DUMP_ROWS", 3000)
+    monkeypatch.setattr(bench, "DUMP_QUAL_MAX", 300_000)            # 3000 records x 150 B: the cut applies
+    fetched = []
+    real_dump = bench.dump_outputs
+
+    def spy(path, out_np, n_reads, tables, emp, suffix=""):
+        fetched.append(([a.copy() for a in out_np], tables.copy(), emp.copy()))
+        real_dump(path, out_np, n_reads, tables, emp, suffix)
+    monkeypatch.setattr(bench, "dump_outputs", spy)
+    dumps = []
+    for k in (2, 5):
+        out = tmp_path / f"steps{k}"
+        d = _run_bench(monkeypatch, bench, ["--reads", "12000", "--steps", str(k), "--warmup", "1", "--no-cpu-baseline", "--dump-outputs", str(out)])
+        assert d["steps"] == k and d["gpu_launches"] == 49 * k and d["verified"] is True
+        files = sorted(os.listdir(out))
+        assert files == sorted(f"{n}.npy" for n in ("rows", "order", "flag", "qual_len", "qual", "bqsr_tables", "empirical_quality"))
+        assert sum(os.path.getsize(out / f) for f in files) <= 64 << 20
+        a = {f[:-4]: np.load(out / f) for f in files}
+        assert all(x.dtype in (np.float32, np.float64) for x in a.values())
+        dumps.append(a)
+    assert dumps[0].keys() == dumps[1].keys() and all(np.array_equal(dumps[0][n], dumps[1][n]) for n in dumps[0])
+    (idx, flag, qoff, qual), tables, emp = fetched[-1]
+    a = dumps[-1]
+    rows = a["rows"].astype(np.int64)
+    assert 0 < rows.size < 3000 and np.all(np.diff(rows) > 0) and a["qual"].size == a["qual_len"].sum() <= 300_000
+    assert np.array_equal(a["order"], idx[rows]) and np.array_equal(a["flag"], flag[rows])
+    assert np.array_equal(a["qual"], np.concatenate([qual[qoff[r]:qoff[r + 1]] for r in rows]))
+    assert np.array_equal(a["bqsr_tables"], tables) and np.array_equal(a["empirical_quality"], emp) and tables.sum() > 0
 
 
 def _rank_main(rank, world, port, out_dir):
