@@ -112,11 +112,9 @@ int qual_presence_update(elp_ctx* c, uint64_t first_byte, uint64_t n_bytes) {
 int upload_side_inputs(elp_ctx* c) {
     if (!c->side_dirty) return E_OK;
     const int nc = c->n_contigs;
-    std::vector<const uint8_t*> rp(nc), np(nc), hp(nc); std::vector<const int32_t*> sp(nc);
-    for (int i = 0; i < nc; i++) { rp[i] = c->d_ref[i]; np[i] = c->d_refnib_raw[i] ? c->d_refnib_raw[i] + 32 : nullptr; hp[i] = c->d_refhot_raw[i] ? c->d_refhot_raw[i] + REFHOT_PAD : nullptr; sp[i] = c->d_sites[i]; }
+    std::vector<const uint8_t*> hp(nc); std::vector<const int32_t*> sp(nc);
+    for (int i = 0; i < nc; i++) { hp[i] = c->d_refhot_raw[i] ? c->d_refhot_raw[i] + REFHOT_PAD : nullptr; sp[i] = c->d_sites[i]; }
     if (nc) {
-        CUDA_TRY(c, cudaMemcpyAsync(c->d_ref_ptrs, rp.data(), nc * sizeof(void*), cudaMemcpyHostToDevice, c->stream));
-        CUDA_TRY(c, cudaMemcpyAsync(c->d_refnib_ptrs, np.data(), nc * sizeof(void*), cudaMemcpyHostToDevice, c->stream));
         CUDA_TRY(c, cudaMemcpyAsync(c->d_refhot_ptrs, hp.data(), nc * sizeof(void*), cudaMemcpyHostToDevice, c->stream));
         CUDA_TRY(c, cudaMemcpyAsync(c->d_ref_len, c->ref_len.data(), nc * 8, cudaMemcpyHostToDevice, c->stream));
         CUDA_TRY(c, cudaMemcpyAsync(c->d_site_ptrs, sp.data(), nc * sizeof(void*), cudaMemcpyHostToDevice, c->stream));
@@ -172,7 +170,7 @@ int elp_create(const elp_config* cfg, elp_ctx** out) {
     const int nc = std::max(1, c->n_contigs), nr = std::max(1, c->n_rg);
     bool ok = cudaMalloc(&c->d_rg_lib, nr * 4) == cudaSuccess && cudaMalloc(&c->d_rg_cov, nr * 4) == cudaSuccess && cudaMalloc(&c->d_contig_len, nc * 4) == cudaSuccess &&
               cudaMalloc(&c->d_ranges, sizeof(DeviceRanges)) == cudaSuccess && cudaMalloc(&c->d_err, 4) == cudaSuccess &&
-              cudaMalloc(&c->d_ref_ptrs, nc * sizeof(void*)) == cudaSuccess && cudaMalloc(&c->d_refnib_ptrs, nc * sizeof(void*)) == cudaSuccess && cudaMalloc(&c->d_refhot_ptrs, nc * sizeof(void*)) == cudaSuccess &&
+              cudaMalloc(&c->d_refhot_ptrs, nc * sizeof(void*)) == cudaSuccess &&
               cudaMalloc(&c->d_bq_small, 512 * 4) == cudaSuccess && cudaMalloc(&c->d_qpresent, 16) == cudaSuccess && cudaMalloc(&c->d_ref_len, nc * 8) == cudaSuccess &&
               cudaMalloc(&c->d_site_ptrs, nc * sizeof(void*)) == cudaSuccess && cudaMalloc(&c->d_n_sites, nc * 8) == cudaSuccess &&
               cudaMalloc(&c->d_tables, std::max<size_t>(16, c->geom.cells() * 2 * sizeof(int64_t))) == cudaSuccess;
@@ -183,7 +181,7 @@ int elp_create(const elp_config* cfg, elp_ctx** out) {
     cudaMemset(c->d_qpresent, 0, 16);
     c->n_qual = c->n_seq = ARENA_FRONT_PAD;
     cudaMemset(c->d_tables, 0, std::max<size_t>(16, c->geom.cells() * 2 * sizeof(int64_t)));
-    c->d_ref.assign(c->n_contigs, nullptr); c->d_refnib_raw.assign(c->n_contigs, nullptr); c->d_refhot_raw.assign(c->n_contigs, nullptr); c->ref_len.assign(c->n_contigs, 0);
+    c->d_refhot_raw.assign(c->n_contigs, nullptr); c->ref_len.assign(c->n_contigs, 0);
     c->d_sites.assign(c->n_contigs, nullptr); c->n_sites.assign(c->n_contigs, 0);
     if ((e = cudaGetLastError()) != cudaSuccess) { c->err = std::string("elp_create: ") + cudaGetErrorString(e); return bail(ELP_ECUDA); }
     *out = c;
@@ -194,14 +192,12 @@ void elp_destroy(elp_ctx* c) {
     if (!c) return;
     cudaSetDevice(c->device);
     if (c->stream) cudaStreamSynchronize(c->stream);
-    for (auto p : c->d_ref) if (p) cudaFree(p);
-    for (auto p : c->d_refnib_raw) if (p) cudaFree(p);
     for (auto p : c->d_refhot_raw) if (p) cudaFree(p);
     for (auto p : c->d_sites) if (p) cudaFree(p);
     for (auto p : c->d_regions) if (p) cudaFree(p);
     if (c->d_region_ptrs) cudaFree((void*)c->d_region_ptrs);
     if (c->d_n_regions) cudaFree(c->d_n_regions);
-    void* singles[] = {c->d_rg_lib, c->d_rg_cov, c->d_contig_len, c->d_ranges, c->d_err, (void*)c->d_ref_ptrs, (void*)c->d_refnib_ptrs, (void*)c->d_refhot_ptrs, c->d_bq_small, c->d_qpresent, c->d_ref_len, (void*)c->d_site_ptrs, c->d_n_sites, c->d_tables,
+    void* singles[] = {c->d_rg_lib, c->d_rg_cov, c->d_contig_len, c->d_ranges, c->d_err, (void*)c->d_refhot_ptrs, c->d_bq_small, c->d_qpresent, c->d_ref_len, (void*)c->d_site_ptrs, c->d_n_sites, c->d_tables,
                        c->d_lut, c->d_clut, c->d_rowtab, c->d_cov_exists, c->d_opt_ctr, c->d_opt_hist, c->d_opt_ovf, c->d_opt_small, c->d_rg_names, c->d_rg_name_off, c->ws.ghist, c->ws.gofs, c->ws.counters, c->ws.status};
     for (void* p : singles) if (p) cudaFree(p);
     c->refid.release(); c->pos.release(); c->nref.release(); c->pnext.release(); c->tlen.release(); c->rg.release(); c->flag.release(); c->mapq.release(); c->optf.release(); c->s_optf.release();
@@ -254,11 +250,7 @@ int elp_set_reference(elp_ctx* c, int32_t contig, const uint8_t* bases, uint64_t
     if (!c) return ELP_EINVAL;
     cudaSetDevice(c->device);
     if (contig < 0 || contig >= c->n_contigs) return c->fail(E_INVAL, "elp_set_reference: contig %d out of range", contig);
-    if (c->d_ref[contig]) { cudaFree(c->d_ref[contig]); c->d_ref[contig] = nullptr; }
-    CUDA_TRY(c, cudaMalloc(&c->d_ref[contig], n + 16));
-    CUDA_TRY(c, cudaMemcpy(c->d_ref[contig], bases, n, cudaMemcpyHostToDevice));
-    c->ref_len[contig] = n; c->side_dirty = true;
-    return pack_reference(c, contig);
+    return pack_reference(c, contig, bases, n);
 }
 
 int elp_set_known_sites(elp_ctx* c, int32_t contig, const int32_t* se, uint64_t n_intervals, int already_flat) {

@@ -1,15 +1,20 @@
 // bqsr_gather.cu -- BQSR covariate gather on the device (replaces (*BaseRecalibrator).Recalibrate,
 // filters/bqsr.go:467-551, with the read clipping of filters/utils.go:130-534).
 //
-// Two kernels over the reads in output (coordinate) order:
+// The fast path (bqsr_prep2_kernel, bqsr_count_kernel: bqsr_count.inl) takes the reads whose clipping has a closed form when
+// the QUAL alphabet is small.  The general kernels below take every read it refuses, or all reads when it does not apply,
+// in output (coordinate) order:
 //   bqsr_prep_kernel   one THREAD per read: recalibrateAln eligibility (:225-244), hardClipAdaptorSequence and
 //                      hardClipSoftClippedBases on a private copy of the CIGAR (utils.go:148-534), the known-sites
 //                      intersection and its read coordinates (calculateSkipSlice :389-414).  The serial, branchy CIGAR
-//                      surgery runs 32 reads per warp instead of one; the result is a 32-byte descriptor per read.
-//   bqsr_count_kernel  one WARP per read, one lane per base: mismatch vs reference (computeSnpEvents :254-285), cycle
-//                      (:376-387) and 2-mer context (:64-146,312-362) covariates, and the table updates.  Observation
-//                      counters of the frequent QUAL values are privatised in shared memory per CTA (persistent CTAs,
-//                      flushed once with 64-bit atomics); mismatches (rare) and infrequent QUAL values go to the global table.
+//                      surgery runs 32 reads per warp instead of one; the result is a 48-byte descriptor per read.
+//   gen_list_kernel    lists the eligible reads that bqsr_chunk_kernel<false> does not take.
+//   bqsr_chunk_kernel  16 consecutive bases per lane: mismatch vs reference (computeSnpEvents :254-285), cycle (:376-387) and
+//                      2-mer context (:64-146,312-362) covariates, and the table updates.  Observation and mismatch counters
+//                      of the frequent QUAL values are privatised in shared memory per CTA (persistent CTAs, flushed once
+//                      with 64-bit atomics); infrequent QUAL values go to the global table.  <false> takes the reads whose
+//                      clipped CIGAR is one M run inside the contig; <true> the listed ones (insertions / deletions, more
+//                      than 4 known-site ranges, cycles beyond --max-cycle, bases past the contig end).
 // Kept bases keep their original alignment under hard clipping, so reference positions come from the ORIGINAL CIGAR
 // offset by the clip start; only the known-sites mask needs the clipped CIGAR (its coordinate mapping has quirks).
 // Table layout: dense int64 [n_cov][94][1 + (2*max_cycle+1) + 16][2] = (observations, mismatches); the
@@ -24,7 +29,6 @@ namespace {
 
 constexpr int MAXC = 64;        // CIGAR operations per read handled by the kernel
 constexpr int MAXIT = 16;       // 32*MAXIT = 512 bases per clipped read (cycles beyond max_cycle=500 are an error anyway)
-constexpr int WARPS_PER_BLOCK = 8;
 
 __device__ __forceinline__ int op_of(uint32_t c) { return (int)(c & 15); }
 __device__ __forceinline__ int len_of(uint32_t c) { return (int)(c >> 4); }
@@ -170,7 +174,7 @@ struct __align__(16) ReadDesc {
     uint32_t ovf;             // slot of the 512-bit skip bitmask when more than 4 known-site ranges hit the read
     uint16_t skip[4][2];      // inclusive [first,last] clipped read coordinates masked by known sites
 };                            // 48 bytes = three 16-byte loads: location | scalars | skip ranges
-constexpr uint8_t DF_REVERSED = 1, DF_LAST = 2, DF_SINGLE_M = 4, DF_SKIP_OVF = 8, DF_LEAN = 16, DF_CHUNKG = 32;   // DF_CHUNKG: chunk kernel with a per-lane CIGAR walk
+constexpr uint8_t DF_REVERSED = 1, DF_LAST = 2, DF_SINGLE_M = 4, DF_SKIP_OVF = 8, DF_LEAN = 16;
 constexpr int OVF_WORDS = 16;   // 512 bits
 
 struct GatherArgs {
@@ -180,13 +184,11 @@ struct GatherArgs {
     const uint32_t* cigar; const uint8_t *seq, *qual;
     const int32_t* rg_cov; int n_rg;
     const int32_t* contig_len; int n_contigs;
-    const uint8_t* const* ref; const uint64_t* ref_len;
+    const uint8_t* const* refhot; const uint64_t* ref_len;   // per contig: one-hot reference nibbles (A/C/G/T -> 1/2/4/8, else 0), low nibble first
     const int32_t* const* sites; const uint64_t* n_sites;
     TableGeom geom; unsigned long long* tables; uint32_t* err;
     ReadDesc* desc; uint32_t* ovf_bits; uint32_t* ovf_count; uint32_t ovf_cap;
-    const uint8_t* const* refnib;    // per contig: reference base codes, 4 bits per base, low nibble first
-    uint32_t* gen_list; uint32_t* gen_count;   // [0]: reads for the warp-per-read fallback kernel, list grows up from gen_list[0]
-    uint32_t* cg_list;                         // [1] of gen_count: insertion/deletion reads for the chunk kernel's GEN variant
+    uint32_t* gen_list; uint32_t* gen_count;   // reads for the chunk kernel's GEN variant
     int lanes_per_read;              // chunk kernel: lanes (16-base chunks) reserved per read
     // shared-memory privatisation: observation counters of the frequent QUAL values live in shared memory
     int8_t qslot[94]; uint8_t slot_q[94]; int n_slots, Lc;
@@ -305,21 +307,18 @@ __global__ void __launch_bounds__(128) bqsr_prep_kernel(GatherArgs A) {
             d.flags |= DF_SKIP_OVF; d.ovf = slot;
         }
     }
-    // chunk kernel: one M run, every cycle inside --max-cycle (|cycle| <= L), inside the contig, fits the lanes of a read
-    if (!A.in_list && (d.flags & DF_SINGLE_M) && !(d.flags & DF_SKIP_OVF) && L <= A.geom.max_cycle && L <= CHUNK * A.lanes_per_read &&
+    // chunk kernel without a list: one M run, every cycle inside --max-cycle (|cycle| <= L), inside the contig.  Every read fits
+    // the lanes of a read: L <= min(512, lseq_max) <= CHUNK * lanes_per_read.
+    if (!A.in_list && (d.flags & DF_SINGLE_M) && !(d.flags & DF_SKIP_OVF) && L <= A.geom.max_cycle &&
         (uint64_t)(a.pos - 1) + (uint64_t)L <= A.ref_len[refid]) d.flags |= DF_LEAN;
-    else if (!(d.flags & DF_SKIP_OVF) && L <= A.geom.max_cycle && L <= CHUNK * A.lanes_per_read) d.flags |= DF_CHUNKG;
     done();
 }
 
-// ---------------------------------------------------------------- shared helpers of the two counting kernels
-// base code of a BAM nibble: A C G T -> 0..3, everything else 8 (bit 3 = "not ACGT", bqsr.go:509)
-__device__ __forceinline__ uint32_t nib_code(uint32_t nib) { return (uint32_t)((0x8888888388828108ull >> (4 * nib)) & 0xfull); }
-
-// rare per-base events, out of line: QUAL without a shared-memory slot, QUAL > 93, base past the contig end
-__device__ __noinline__ void count_rare(const GatherArgs& A, int cov, int q, int cyc, uint32_t ctx, bool okc, uint32_t snp, bool past_end, uint32_t* errbits) {
-    if (q > 93) { *errbits |= DERR_QUAL_RANGE; return; }
-    if (past_end) { *errbits |= DERR_REFEND; return; }
+// rare per-base events, out of line: QUAL without a shared-memory slot, QUAL > 93, a cycle beyond --max-cycle
+// (checkCycleCovariate, bqsr.go:364-369)
+__device__ __noinline__ void count_rare(const GatherArgs& A, int cov, int q, int cyc, uint32_t ctx, bool okc, uint32_t snp, uint32_t* errbits) {
+    const uint32_t e = (q > 93 ? DERR_QUAL_RANGE : 0u) | (cyc > A.geom.max_cycle || cyc < -A.geom.max_cycle ? DERR_CYCLE : 0u);
+    if (e) { *errbits |= e; return; }
     atomicAdd(A.tables + 2 * A.geom.idx(cov, q, A.geom.col_cycle(cyc)), 1ull);
     if (okc) atomicAdd(A.tables + 2 * A.geom.idx(cov, q, A.geom.col_ctx((int)ctx)), 1ull);
     if (snp) {
@@ -338,7 +337,7 @@ __device__ __forceinline__ void reds_add(uint32_t a, uint32_t v) { asm volatile(
 // reads per step; lane (r, c) owns bases [16c, 16c+16) of read r.  Everything per base is SIMD inside 32/64-bit words:
 //   QUAL    16 bytes  (unaligned 16-byte window out of two aligned 128-bit loads)
 //   SEQ     16 BAM nibbles -> base codes 0..3 / 8 by bit arithmetic, 4 bits per base
-//   REF     16 nibbles of pre-packed reference codes (pack_reference): mismatch = XOR
+//   REF     16 one-hot reference nibbles (pack_reference); the read's BAM nibbles are one-hot for A/C/G/T too: mismatch = XOR
 //   context previous base in sequencing direction by shifting the code word one nibble (edge nibble from the neighbour lane)
 //   masks   counted / context-valid / mismatch / known-site flags as one bit per nibble
 // leaving ~14 instructions per base for the two shared-memory increments (cycle, context).  The cycle column of a
@@ -349,7 +348,10 @@ struct ChunkSmem { uint32_t obs, mis, qslot; };   // shared-window byte addresse
 #ifndef CHUNK_MINB
 #define CHUNK_MINB 4
 #endif
-template <bool GEN>   // GEN: reads come from a list and may contain insertions / deletions (reference window per lane from the CIGAR)
+// GEN: every eligible read that is not DF_LEAN, from a list.  The reference window of a lane comes from a walk of the CIGAR
+// (insertions / deletions, bases past the contig end); known sites may come as the 512-bit mask (DF_SKIP_OVF); a read longer
+// than --max-cycle takes its cycles past the shared-memory rows, so all its counted bases go to the global table.
+template <bool GEN>
 __global__ void __launch_bounds__(256, CHUNK_MINB) bqsr_chunk_kernel(GatherArgs A, const uint32_t* __restrict__ list, uint32_t n_list) {
     extern __shared__ uint32_t sm_tab[];
     // QUAL -> row of the CTA's tables: bits 0..5 = shared-memory slot, or n_slots = the trash row (updates that must not
@@ -403,19 +405,20 @@ __global__ void __launch_bounds__(256, CHUNK_MINB) bqsr_chunk_kernel(GatherArgs 
         nloc = make_uint4(0, 0, 0, 0); nsc = nloc;
         if (lane_used && inext < n_items) { nread = read_of(inext); nloc = __ldg(dbase + 3 * nread); nsc = __ldg(dbase + 3 * nread + 1); }
         const uint32_t flags = sc.z & 0xff;
-        const int L = (have && (flags & (GEN ? DF_CHUNKG : DF_LEAN))) ? (int)(sc.y >> 16) : 0;   // 0: nothing to do for this lane group
-        const int i0 = c * CHUNK, nb = min(max(L - i0, 0), CHUNK);                                // bases of this chunk
+        const int L = (have && (GEN || (flags & DF_LEAN))) ? (int)(sc.y >> 16) : 0;   // 0: nothing to do for this lane group
+        const int i0 = c * CHUNK, nb = min(max(L - i0, 0), CHUNK);                      // bases of this chunk
         const bool rev = flags & DF_REVERSED;
         // ---- loads ----
         uint32_t Q[4] = {0, 0, 0, 0};
-        unsigned long long C = 0, R = 0, pastf = 0;
+        unsigned long long C = 0, X = 0, pastf = 0;   // X: read nibbles XOR reference nibbles, non-zero where they differ
         if (nb > 0) {
             const uint64_t qloc = ((uint64_t)loc.y << 32) | loc.x, nl = ((uint64_t)loc.w << 32) | loc.z;
             const uint32_t refid = (uint32_t)(qloc >> 40);
             load16_unaligned(A.qual + (qloc & ((1ull << 40) - 1)) + (uint64_t)i0, Q);
             const unsigned long long nibs = load16_nibbles_bam(A.seq, nl + (uint64_t)i0);
             C = (unsigned long long)codes_of((uint32_t)nibs) | ((unsigned long long)codes_of((uint32_t)(nibs >> 32)) << 32);
-            if (!GEN) R = load16_nibbles_le(A.refnib[refid], (uint64_t)((int64_t)(int32_t)sc.x - 1 + i0));
+            unsigned long long R = 0;
+            if (!GEN) R = load16_nibbles_le(A.refhot[refid], (uint64_t)((int64_t)(int32_t)sc.x - 1 + i0));
             else {
                 // computeSnpEvents (bqsr.go:254-285) over the ORIGINAL alignment (kept bases keep their positions under hard
                 // clipping): find the operation holding the chunk's first base; a chunk inside one M run is one window load,
@@ -430,9 +433,9 @@ __global__ void __launch_bounds__(256, CHUNK_MINB) bqsr_chunk_kernel(GatherArgs 
                 }
                 const int64_t reflen = (int64_t)A.ref_len[refid];
                 const bool mtype = opk == 0 || opk == 7 || opk == 8;
-                if (mtype && oi0 + nb <= ri + oplen && j + (oi0 - ri) + nb <= reflen) R = load16_nibbles_le(A.refnib[refid], (uint64_t)(j + (oi0 - ri)));
+                if (mtype && oi0 + nb <= ri + oplen && j + (oi0 - ri) + nb <= reflen) R = load16_nibbles_le(A.refhot[refid], (uint64_t)(j + (oi0 - ri)));
                 else {
-                    const uint8_t* rn = A.refnib[refid];
+                    const uint8_t* rh = A.refhot[refid];
                     int rem = opk < 0 ? 0 : ri + oplen - oi0;                   // bases left in the current operation
                     int64_t jj = j + (mtype ? (oi0 - ri) : 0);
                     bool m = mtype;
@@ -443,10 +446,10 @@ __global__ void __launch_bounds__(256, CHUNK_MINB) bqsr_chunk_kernel(GatherArgs 
                             if (o == 2 || o == 3) { jj += ln; continue; }
                             if (cons_read(o)) { rem = ln; m = (o == 0 || o == 7 || o == 8); }
                         }
-                        unsigned long long rc = (C >> (4 * b)) & 15ull;         // no reference base (insertion): never a mismatch
+                        unsigned long long rc = (nibs >> (4 * b)) & 15ull;      // no reference base (insertion): never a mismatch
                         if (m) {
                             if (jj >= reflen) pastf |= 1ull << (4 * b);
-                            else rc = (unsigned long long)((__ldg(rn + (jj >> 1)) >> (4 * (int)(jj & 1))) & 15u);
+                            else rc = (unsigned long long)((__ldg(rh + (jj >> 1)) >> (4 * (int)(jj & 1))) & 15u);
                             jj++;
                         }
                         R |= rc << (4 * b);
@@ -454,6 +457,7 @@ __global__ void __launch_bounds__(256, CHUNK_MINB) bqsr_chunk_kernel(GatherArgs 
                     }
                 }
             }
+            X = nibs ^ R;
         }
         if (nb < CHUNK) { const unsigned long long inlen = range16(0, nb - 1); C = (C & (inlen * 15ull)) | ((ONES & ~inlen) << 3); }   // codes past the read end: 8
         // ---- low-quality tails (computeStrandedClippedSeq, bqsr.go:312-331): first / last base with QUAL > 2 ----
@@ -479,10 +483,16 @@ __global__ void __launch_bounds__(256, CHUNK_MINB) bqsr_chunk_kernel(GatherArgs 
             const uint32_t skv[4] = {sk.x, sk.y, sk.z, sk.w};
 #pragma unroll
             for (int t = 0; t < 4; t++) if (t < (int)n_skip) skipf |= range16((int)(skv[t] & 0xffff) - i0, (int)(skv[t] >> 16) - i0);
+        } else if (GEN && (flags & DF_SKIP_OVF)) {
+            // more than 4 ranges: the chunk's 16 bits of the read's 512-bit mask (i0 is a multiple of 16: one word), one flag per nibble
+            unsigned long long x = (__ldg(A.ovf_bits + (size_t)sc.w * OVF_WORDS + (i0 >> 5)) >> (i0 & 31)) & 0xffffull;
+            x = (x | x << 24) & 0x000000FF000000FFull;
+            x = (x | x << 12) & 0x000F000F000F000Full;
+            x = (x | x << 6) & 0x0303030303030303ull;
+            skipf = (x | x << 3) & ONES;
         }
         const unsigned long long counted = ~(C >> 3) & ONES & ~skipf;                             // ACGT, inside the read, not a known site (QUAL >= 6 via the slot table)
         const unsigned long long okc = counted & ~((Pn | C) >> 3) & range16(wlo - i0, whi - i0);
-        const unsigned long long X = C ^ R;
         const unsigned long long snpf = (X | (X >> 1) | (X >> 2) | (X >> 3)) & counted;         // computeSnpEvents, bqsr.go:254-285
         if (GEN && (pastf & counted)) errbits |= DERR_REFEND;                                   // a counted base beyond the end of its contig
         if (counted) {
@@ -495,24 +505,28 @@ __global__ void __launch_bounds__(256, CHUNK_MINB) bqsr_chunk_kernel(GatherArgs 
         const uint32_t cnt_w[2] = {(uint32_t)counted, (uint32_t)(counted >> 32)}, okc_w[2] = {(uint32_t)okc, (uint32_t)(okc >> 32)};
         const uint32_t ctx_w[2] = {(uint32_t)ctxw, (uint32_t)(ctxw >> 32)};
         const uint32_t obs_ctx = obs0 + ctx_off;
+        // a read longer than --max-cycle has cycles beyond the shared-memory rows (|cycle| <= Lc): all its counted bases take the slow tail
+        const bool global_only = GEN && L > A.geom.max_cycle;
         uint32_t racc = 0;
-        int ci = ci0;
+        if (!global_only) {
+            int ci = ci0;
 #pragma unroll
-        for (int j = 0; j < CHUNK; j++) {
-            // no predicates and no branches: a base that is not counted adds 0, a QUAL without a slot adds to the trash row
-            const uint32_t q = (Q[j >> 2] >> (8 * (j & 3))) & 0xffu;
-            const uint32_t lut = lds_u8(S.qslot + q);
-            const uint32_t roff = (lut & 0x3fu) * row_bytes;
-            const uint32_t a1 = obs0 + roff + (uint32_t)(ci + (ci >> 4)) * 4u;
-            const uint32_t nib4 = (j & 7) == 0 ? ((ctx_w[j >> 3] << 2) & 0x3cu) : ((ctx_w[j >> 3] >> (4 * (j & 7) - 2)) & 0x3cu);
-            const uint32_t a2 = obs_ctx + roff + nib4;
-            reds_add(a1, (cnt_w[j >> 3] >> (4 * (j & 7))) & 1u);
-            reds_add(a2, (okc_w[j >> 3] >> (4 * (j & 7))) & 1u);
-            racc |= lut;
-            ci += inc;
+            for (int j = 0; j < CHUNK; j++) {
+                // no predicates and no branches: a base that is not counted adds 0, a QUAL without a slot adds to the trash row
+                const uint32_t q = (Q[j >> 2] >> (8 * (j & 3))) & 0xffu;
+                const uint32_t lut = lds_u8(S.qslot + q);
+                const uint32_t roff = (lut & 0x3fu) * row_bytes;
+                const uint32_t a1 = obs0 + roff + (uint32_t)(ci + (ci >> 4)) * 4u;
+                const uint32_t nib4 = (j & 7) == 0 ? ((ctx_w[j >> 3] << 2) & 0x3cu) : ((ctx_w[j >> 3] >> (4 * (j & 7) - 2)) & 0x3cu);
+                const uint32_t a2 = obs_ctx + roff + nib4;
+                reds_add(a1, (cnt_w[j >> 3] >> (4 * (j & 7))) & 1u);
+                reds_add(a2, (okc_w[j >> 3] >> (4 * (j & 7))) & 1u);
+                racc |= lut;
+                ci += inc;
+            }
         }
         // slow tail: mismatches (sparse) and, if some base of the chunk has a QUAL without a shared-memory slot, all counted bases
-        unsigned long long later = (racc & 0x80u) ? counted : snpf;
+        unsigned long long later = (global_only || (racc & 0x80u)) ? counted : snpf;
         while (later) {
             const int j = (__ffsll((long long)later) - 1) >> 2;
             later &= ~(15ull << (4 * j));
@@ -522,12 +536,13 @@ __global__ void __launch_bounds__(256, CHUNK_MINB) bqsr_chunk_kernel(GatherArgs 
             const int cj = ci0 + j * inc;
             const uint32_t ctx = (uint32_t)((ctxw >> (4 * j)) & 15ull);
             const bool ok = (okc >> (4 * j)) & 1ull, snp = (snpf >> (4 * j)) & 1ull;
-            if ((lut & 0x40u) || (!(lut & 0x80u) && !snp)) continue;   // QUAL < 6: not counted; slotted match: done in the fast loop
-            if (!(lut & 0x80u)) {     // a mismatch (sparse, ~0.5 % of bases) on the CTA's second table
+            const bool slotted = !global_only && !(lut & 0x80u);
+            if ((lut & 0x40u) || (slotted && !snp)) continue;   // QUAL < 6: not counted; slotted match: done in the fast loop
+            if (slotted) {     // a mismatch (sparse, ~0.5 % of bases) on the CTA's second table
                 const uint32_t mrow = S.mis + (cov * (uint32_t)rows + (lut & 0x3fu)) * row_bytes;
                 reds_inc(mrow + (uint32_t)(cj + (cj >> 4)) * 4u);
                 if (ok) reds_inc(mrow + ctx_off + ctx * 4u);
-            } else count_rare(A, (int)cov, (int)q, cj - Lc, ctx, ok, snp ? 1u : 0u, false, &errbits);
+            } else count_rare(A, (int)cov, (int)q, cj - Lc, ctx, ok, snp ? 1u : 0u, &errbits);
         }
         }
         }
@@ -549,184 +564,24 @@ __global__ void __launch_bounds__(256, CHUNK_MINB) bqsr_chunk_kernel(GatherArgs 
     }
 }
 
-// reference bases -> 4-bit codes (baseToIntMap, bqsr.go:247-252: A/a/* C/c G/g T/t -> 0..3, everything else 8), low nibble first
-__global__ void __launch_bounds__(256) ref_pack_kernel(const uint8_t* __restrict__ ref, uint64_t n, uint8_t* __restrict__ out, uint64_t n_out) {
-    const uint64_t t = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= n_out) return;
-    uint32_t v = 0;
-#pragma unroll
-    for (int h = 0; h < 2; h++) {
-        const uint64_t j = 2 * t + h; uint32_t cd = 8;
-        if (j < n) { const uint8_t b = ref[j]; if (b == 'A' || b == 'a' || b == '*') cd = 0; else if (b == 'C' || b == 'c') cd = 1; else if (b == 'G' || b == 'g') cd = 2; else if (b == 'T' || b == 't') cd = 3; }
-        v |= cd << (4 * h);
-    }
-    out[t] = (uint8_t)v;
-}
-
-// work lists of the eligible reads that are not DF_LEAN: DF_CHUNKG reads (insertions / deletions) for the chunk kernel's GEN
-// variant, everything else for the warp-per-read fallback.  One global atomic per block and list.
+// work list of the eligible reads that are not DF_LEAN, for the chunk kernel's GEN variant.  One global atomic per block.
 __global__ void __launch_bounds__(256) gen_list_kernel(GatherArgs A) {
-    __shared__ uint32_t s_cnt[2], s_base[2];
-    if (threadIdx.x < 2) s_cnt[threadIdx.x] = 0;
+    __shared__ uint32_t s_cnt, s_base;
+    if (threadIdx.x == 0) s_cnt = 0;
     __syncthreads();
     const uint64_t tix = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
     const bool in = tix < (A.in_list ? (uint64_t)A.n_in : A.n);
     const uint64_t k = in ? (A.in_list ? (uint64_t)A.in_list[tix] : tix) : 0;
-    int which = -1;
-    if (in) { const uint4 sc = __ldg(reinterpret_cast<const uint4*>(A.desc) + 3 * k + 1); if ((sc.y >> 16) != 0 && !(sc.z & DF_LEAN)) which = (sc.z & DF_CHUNKG) ? 1 : 0; }
-    uint32_t wbase = 0, before = 0;
-#pragma unroll
-    for (int l = 0; l < 2; l++) {
-        const unsigned b = __ballot_sync(FULL_MASK, which == l);
-        uint32_t wb = 0;
-        if (b && lane_id() == 0) wb = atomicAdd(&s_cnt[l], (uint32_t)__popc(b));
-        wb = __shfl_sync(FULL_MASK, wb, 0);
-        if (which == l) { wbase = wb; before = __popc(b & lanemask_lt()); }
-    }
+    bool want = false;
+    if (in) { const uint4 sc = __ldg(reinterpret_cast<const uint4*>(A.desc) + 3 * k + 1); want = (sc.y >> 16) != 0 && !(sc.z & DF_LEAN); }
+    const unsigned b = __ballot_sync(FULL_MASK, want);
+    uint32_t wb = 0;
+    if (b && lane_id() == 0) wb = atomicAdd(&s_cnt, (uint32_t)__popc(b));
+    wb = __shfl_sync(FULL_MASK, wb, 0);
     __syncthreads();
-    if (threadIdx.x < 2 && s_cnt[threadIdx.x]) s_base[threadIdx.x] = atomicAdd(A.gen_count + threadIdx.x, s_cnt[threadIdx.x]);
+    if (threadIdx.x == 0 && s_cnt) s_base = atomicAdd(A.gen_count, s_cnt);
     __syncthreads();
-    if (which == 0) A.gen_list[s_base[0] + wbase + before] = (uint32_t)k;
-    if (which == 1) A.cg_list[s_base[1] + wbase + before] = (uint32_t)k;
-}
-
-// ---------------------------------------------------------------- kernel C: one warp per read, one lane per base
-// (insertions / deletions, cycles beyond --max-cycle, > 4 known-site ranges, reads running off their contig)
-__global__ void __launch_bounds__(WARPS_PER_BLOCK * 32, 2048 / (WARPS_PER_BLOCK * 32 * 2)) bqsr_general_kernel(GatherArgs A, uint32_t n_gen) {
-    extern __shared__ uint32_t sm_tab[];
-    __shared__ uint8_t sm_refcode[256];   // baseToIntMap (bqsr.go:247-252): A/a/* C/c G/g T/t -> 0..3, everything else 8
-    __shared__ int8_t sm_qslot[256];      // QUAL -> shared-memory slot, -1 = none (and for QUAL > 93)
-    const unsigned lane = lane_id(), w = threadIdx.x >> 5;
-    const int Lc = A.Lc, ncols_s = 2 * Lc + 1 + 16, max_cycle = A.geom.max_cycle;    // this kernel's rows are not skewed
-    const int cells = A.geom.n_cov * A.n_slots * ncols_s;
-    uint32_t* sm_mis = sm_tab + cells;
-    for (int i = threadIdx.x; i < 2 * cells; i += blockDim.x) sm_tab[i] = 0;
-    {
-        const int b = threadIdx.x; uint8_t c = 8;
-        if (b == 'A' || b == 'a' || b == '*') c = 0; else if (b == 'C' || b == 'c') c = 1; else if (b == 'G' || b == 'g') c = 2; else if (b == 'T' || b == 't') c = 3;
-        sm_refcode[b] = c;
-        sm_qslot[b] = b < 94 ? A.qslot[b] : (int8_t)-1;
-    }
-    __syncthreads();
-    const uint64_t stride = (uint64_t)gridDim.x * WARPS_PER_BLOCK;
-    for (uint64_t gi = (uint64_t)blockIdx.x * WARPS_PER_BLOCK + w; gi < n_gen; gi += stride) {
-        const uint64_t k = A.gen_list[gi];
-        const uint4* dp = reinterpret_cast<const uint4*>(A.desc) + 3 * k;
-        const uint4 d0 = __ldg(dp + 1);
-        const int L = (int)(d0.y >> 16);
-        if (L == 0) continue;
-        const uint4 d1 = __ldg(dp + 2);
-        const int c_pos = (int)d0.x, c_s0 = (int)(d0.y & 0xffff);
-        const uint32_t flags = d0.z & 0xff, cov = (d0.z >> 8) & 0xff, n_skip = (d0.z >> 16) & 0xff;
-        const int reversed = (flags & DF_REVERSED) ? 1 : 0, last = (flags & DF_LAST) ? 1 : 0;
-        const int32_t refid = A.refid[k];
-        const uint8_t* qualp = A.qual + A.qual_off[k] + c_s0;
-        const uint8_t* seqp = A.seq + A.seq_off[k];
-        const uint8_t* ref = A.ref[refid]; const int64_t reflen = (int64_t)A.ref_len[refid];
-        const int nit = (L + 31) >> 5;
-        // ---- general path: insertions / deletions, or a cycle beyond --max-cycle somewhere in the read ----
-        // low-quality tails (computeStrandedClippedSeq, bqsr.go:312-331): first / last base with QUAL > 2
-        int leftPos = L, rightPos = -1;
-        for (int it = 0; it < nit; it++) {
-            const int i = lane + it * 32;
-            const unsigned b = __ballot_sync(FULL_MASK, i < L && qualp[i] > 2);
-            if (b) { if (leftPos == L) leftPos = it * 32 + __ffs(b) - 1; rightPos = it * 32 + 31 - __clz(b); }
-        }
-        // a base has a context iff it and its predecessor in sequencing direction lie inside [leftPos, rightPos]:
-        //   forward: i-1 >= leftPos, i <= rightPos ; reverse: i >= leftPos, i+1 <= rightPos
-        const int wlo = reversed ? leftPos : leftPos + 1, whi = reversed ? rightPos - 1 : rightPos;
-        const uint32_t wspan = (whi >= wlo) ? (uint32_t)(whi - wlo) : 0u;
-        const bool have_win = whi >= wlo;
-        const int rof = 1 - 2 * last, cf = rof + reversed * (L - 1) * rof, inc = (1 - 2 * reversed) * rof;   // prepareCycleCovariates, bqsr.go:376-383
-        const uint32_t cmask = reversed ? 3u : 0u;
-        const uint32_t row0 = cov * (uint32_t)A.n_slots;
-        const bool single_m = (flags & DF_SINGLE_M) != 0;
-        const int64_t j0 = (int64_t)c_pos - 1;
-        // general CIGAR: reference positions from the ORIGINAL alignment (kept bases keep their positions under hard clipping)
-        int32_t pos_orig = 0; uint64_t coff = 0; int nc = 0;
-        if (!single_m) { pos_orig = A.pos[k]; coff = A.cigar_off[k]; nc = (int)A.ncigar[k]; }
-        uint32_t errbits = 0;
-        uint32_t carry = 8;   // code of the base just before this iteration's first lane, in sequencing direction
-        for (int t = 0; t < nit; t++) {
-            const int it = reversed ? nit - 1 - t : t;                   // walk in sequencing direction
-            const int i = lane + it * 32;
-            const bool in = i < L;
-            const int ic = in ? i : L - 1;
-            const int oi = c_s0 + ic;
-            const uint32_t sb = seqp[oi >> 1];
-            const uint32_t nib = (oi & 1) ? (sb & 15u) : (sb >> 4);
-            const uint32_t code = in ? nib_code(nib) : 8u;               // read-orientation code
-            const uint32_t q = qualp[ic];
-            // predecessor in sequencing direction: lane-1 (forward) / lane+1 (reverse); across the 32-base boundary via `carry`
-            uint32_t pcode = __shfl_sync(FULL_MASK, code, reversed ? (lane + 1) & 31 : (lane - 1) & 31);
-            if (lane == (reversed ? 31u : 0u)) pcode = carry;
-            carry = __shfl_sync(FULL_MASK, code, reversed ? 0 : 31);
-            // skip mask
-            bool skipped = false;
-            if (n_skip) {
-                const uint32_t sk[4] = {d1.x, d1.y, d1.z, d1.w};
-#pragma unroll
-                for (int r = 0; r < 4; r++) if (r < (int)n_skip) skipped |= ((uint32_t)ic >= (sk[r] & 0xffff)) & ((uint32_t)ic <= (sk[r] >> 16));
-            } else if (flags & DF_SKIP_OVF) skipped = (A.ovf_bits[(size_t)d0.w * OVF_WORDS + (ic >> 5)] >> (ic & 31)) & 1;
-            const bool counted = in & !skipped & !(code & 8) & (q >= 6);   // bqsr.go:506-515
-            if (!__any_sync(FULL_MASK, counted)) continue;
-            if (counted && q > 93) { errbits |= DERR_QUAL_RANGE; }
-            // reference base (computeSnpEvents, bqsr.go:254-285)
-            int64_t jj = -1;
-            if (single_m) jj = j0 + ic;
-            else {
-                const int oi2 = oi; int ri = 0; int64_t j = (int64_t)pos_orig - 1;
-                for (int c = 0; c < nc; c++) {
-                    const uint32_t op = A.cigar[coff + c]; const int o = op_of(op), ln = len_of(op);
-                    if (o == 0 || o == 7 || o == 8) { if (oi2 < ri + ln) { jj = j + (oi2 - ri); break; } ri += ln; j += ln; }
-                    else if (o == 2 || o == 3) j += ln;
-                    else if (o == 1 || o == 4) { if (oi2 < ri + ln) break; ri += ln; }
-                }
-            }
-            uint32_t snp = 0;
-            if (counted && jj >= 0) {
-                if (jj >= reflen) { errbits |= DERR_REFEND; }
-                else snp = sm_refcode[ref[jj]] != code;
-            }
-            const int cyc = cf + ic * inc;
-            const bool badc = (cyc > max_cycle) | (cyc < -max_cycle);                     // checkCycleCovariate :364-369
-            if (counted & badc) errbits |= DERR_CYCLE;
-            const int slot = sm_qslot[q];
-            const bool okc = counted & !(pcode & 8) & have_win & ((uint32_t)(ic - wlo) <= wspan);
-            const uint32_t ctx = ((pcode ^ cmask) & 3u) | (((code ^ cmask) & 3u) << 2);   // key>>4 = prev | cur<<2 (bqsr.go:64-76), complemented for reverse reads
-            if (counted && q <= 93 && !badc) {
-                if (slot >= 0) {
-                    const uint32_t row = (row0 + (uint32_t)slot) * (uint32_t)ncols_s;
-                    atomicAdd(&sm_tab[row + (uint32_t)(cyc + Lc)], 1u);
-                    if (okc) atomicAdd(&sm_tab[row + (uint32_t)(2 * Lc + 1) + ctx], 1u);
-                } else {
-                    atomicAdd(A.tables + 2 * A.geom.idx((int)cov, (int)q, A.geom.col_cycle(cyc)), 1ull);
-                    if (okc) atomicAdd(A.tables + 2 * A.geom.idx((int)cov, (int)q, A.geom.col_ctx((int)ctx)), 1ull);
-                }
-                if (snp) {
-                    if (slot >= 0) {   // mismatches are sparse (~0.5 % of bases): shared atomics on the CTA's second table
-                        const uint32_t row = (row0 + (uint32_t)slot) * (uint32_t)ncols_s;
-                        atomicAdd(&sm_mis[row + (uint32_t)(cyc + Lc)], 1u);
-                        if (okc) atomicAdd(&sm_mis[row + (uint32_t)(2 * Lc + 1) + ctx], 1u);
-                    } else {
-                        atomicAdd(A.tables + 2 * A.geom.idx((int)cov, (int)q, A.geom.col_cycle(cyc)) + 1, 1ull);
-                        if (okc) atomicAdd(A.tables + 2 * A.geom.idx((int)cov, (int)q, A.geom.col_ctx((int)ctx)) + 1, 1ull);
-                    }
-                }
-            }
-        }
-        errbits = __reduce_or_sync(FULL_MASK, errbits);
-        if (errbits && lane == 0) atomicOr(A.err, errbits);
-    }
-    __syncthreads();
-    for (int i = threadIdx.x; i < cells; i += blockDim.x) {
-        const uint32_t v = sm_tab[i], e = sm_mis[i];
-        if (!(v | e)) continue;
-        const int col_s = i % ncols_s, cs = i / ncols_s, slot = cs % A.n_slots, cov = cs / A.n_slots;
-        const int col_g = col_s < 2 * Lc + 1 ? A.geom.col_cycle(col_s - Lc) : A.geom.col_ctx(col_s - (2 * Lc + 1));
-        if (v) atomicAdd(A.tables + 2 * A.geom.idx(cov, A.slot_q[slot], col_g), (unsigned long long)v);
-        if (e) atomicAdd(A.tables + 2 * A.geom.idx(cov, A.slot_q[slot], col_g) + 1, (unsigned long long)e);
-    }
+    if (want) A.gen_list[s_base + wb + __popc(b & lanemask_lt())] = (uint32_t)k;
 }
 
 // QUAL value histogram of a prefix of the QUAL arena: picks which values get shared-memory slots
@@ -756,36 +611,37 @@ __global__ void derive_q_kernel(TableGeom geom, long long* tables) {
 
 }  // namespace
 
-// nibble-packed reference codes of one contig (read by the chunk kernel); 32 bytes of padding on both sides because the
-// kernel reads aligned 16-byte windows around the bases it needs
-int pack_reference(elp_ctx* c, int contig) {
-    const uint64_t n = c->ref_len[contig], n_out = (n + 1) / 2;
-    if (c->d_refnib_raw[contig]) { cudaFree(c->d_refnib_raw[contig]); c->d_refnib_raw[contig] = nullptr; }
-    CUDA_TRY(c, cudaMalloc(&c->d_refnib_raw[contig], n_out + 64));
-    CUDA_TRY(c, cudaMemsetAsync(c->d_refnib_raw[contig], 0x88, n_out + 64, c->stream));
-    if (n_out) {
-        c->launches++;
-        ref_pack_kernel<<<(unsigned)((n_out + 255) / 256), 256, 0, c->stream>>>(c->d_ref[contig], n, c->d_refnib_raw[contig] + 32, n_out);
-        LAUNCH_CHECK(c);
-    }
-    // one-hot nibbles for the count kernel (bqsr_count.inl); REFHOT_PAD bytes in front (windows of reads at the start of a contig and
-    // the shifted window of an insertion start before base 0), 64 behind
+// the reference bases of one contig -> one-hot nibbles, the only device copy of the genome (read by the chunk and count kernels).
+// REFHOT_PAD bytes in front (windows of reads at the start of a contig and the shifted window of an insertion start before
+// base 0), 64 behind.  The bases pass through a device buffer that is freed before the call returns.
+int pack_reference(elp_ctx* c, int contig, const uint8_t* bases, uint64_t n) {
+    const uint64_t n_out = (n + 1) / 2;
     if (c->d_refhot_raw[contig]) { cudaFree(c->d_refhot_raw[contig]); c->d_refhot_raw[contig] = nullptr; }
+    c->ref_len[contig] = 0; c->side_dirty = true;
     CUDA_TRY(c, cudaMalloc(&c->d_refhot_raw[contig], n_out + REFHOT_PAD + 64));
     CUDA_TRY(c, cudaMemsetAsync(c->d_refhot_raw[contig], 0, n_out + REFHOT_PAD + 64, c->stream));
-    if (n_out) {
-        c->launches++;
-        ref_pack_hot_kernel<<<(unsigned)((n_out + 255) / 256), 256, 0, c->stream>>>(c->d_ref[contig], n, c->d_refhot_raw[contig] + REFHOT_PAD, n_out);
-        LAUNCH_CHECK(c);
+    uint8_t* d_bases = nullptr;
+    cudaError_t e = cudaSuccess;
+    if (n) {
+        CUDA_TRY(c, cudaMalloc(&d_bases, n));
+        e = cudaMemcpyAsync(d_bases, bases, n, cudaMemcpyHostToDevice, c->stream);
+        if (e == cudaSuccess) {
+            c->launches++;
+            ref_pack_hot_kernel<<<(unsigned)((n_out + 255) / 256), 256, 0, c->stream>>>(d_bases, n, c->d_refhot_raw[contig] + REFHOT_PAD, n_out);
+            e = cudaGetLastError();
+        }
     }
-    CUDA_TRY(c, cudaStreamSynchronize(c->stream));
+    if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
+    if (d_bases) cudaFree(d_bases);
+    CUDA_TRY(c, e);
+    c->ref_len[contig] = n;
     return E_OK;
 }
 
 namespace {
 
-// the general kernels (prep -> descriptors -> chunk / warp-per-read kernels with shared-memory counters) over all reads (in_list == nullptr)
-// or over the list bqsr_prep2_kernel left for them
+// the general kernels (prep -> descriptors -> chunk kernels with shared-memory counters) over all reads (in_list == nullptr) or over
+// the list bqsr_prep2_kernel left for them
 int gather_general(elp_ctx* c, GatherArgs A, const uint32_t* in_list, uint32_t n_in, double bytes) {
     const uint64_t n = c->n;
     const uint64_t n_work = in_list ? (uint64_t)n_in : n;
@@ -818,15 +674,15 @@ int gather_general(elp_ctx* c, GatherArgs A, const uint32_t* in_list, uint32_t n
     int sms = 148; cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, c->device);
     // descriptors (48 B/read, indexed by read) and the overflow skip bitmasks live in scratch buffers that are free in this phase
     CUDA_TRY(c, c->keys_a.reserve(n * 6 + 8, c->stream));
-    CUDA_TRY(c, c->vals_b.reserve(2 * n + 16, c->stream));
-    A.gen_list = c->vals_b.p; A.cg_list = c->vals_b.p + n + 8;
+    CUDA_TRY(c, c->vals_b.reserve(n + 8, c->stream));
+    A.gen_list = c->vals_b.p;
     A.desc = reinterpret_cast<ReadDesc*>(c->keys_a.p);
     A.ovf_cap = (uint32_t)std::min<uint64_t>(n, (n >> 4) + 4096);
     CUDA_TRY(c, c->vals_a.reserve((size_t)A.ovf_cap * OVF_WORDS + 8, c->stream));
     A.ovf_bits = c->vals_a.p;
-    A.ovf_count = c->scan_tmp.p;   // three u32 (overflow slots, fallback reads, GEN chunk reads), zeroed below
+    A.ovf_count = c->scan_tmp.p;   // two u32 (overflow slots, GEN chunk reads), zeroed below
     A.gen_count = c->scan_tmp.p + 1;
-    CUDA_TRY(c, cudaMemsetAsync(A.ovf_count, 0, 12, c->stream));
+    CUDA_TRY(c, cudaMemsetAsync(A.ovf_count, 0, 8, c->stream));
     c->begin("bqsr_g_prep", (double)n_work * (4 * 7 + 2 + 1 + 8 + 8 + 4 + 48) + (double)c->n_cigar * 4 * ((double)n_work / (double)n));
     bqsr_prep_kernel<<<(unsigned)((n_work + 127) / 128), 128, 0, c->stream>>>(A);
     c->end(); LAUNCH_CHECK(c);
@@ -844,23 +700,14 @@ int gather_general(elp_ctx* c, GatherArgs A, const uint32_t* in_list, uint32_t n
         bqsr_chunk_kernel<false><<<(unsigned)grid, 256, smem, c->stream>>>(A, nullptr, 0);
         c->end(); LAUNCH_CHECK(c);
     }
-    uint32_t cnt2[2] = {0, 0};
-    CUDA_TRY(c, cudaMemcpyAsync(cnt2, A.gen_count, 8, cudaMemcpyDeviceToHost, c->stream));
+    uint32_t n_gen = 0;
+    CUDA_TRY(c, cudaMemcpyAsync(&n_gen, A.gen_count, 4, cudaMemcpyDeviceToHost, c->stream));
     CUDA_TRY(c, cudaStreamSynchronize(c->stream));
-    const uint32_t n_gen = cnt2[0], n_cg = cnt2[1];
-    if (n_cg) {
-        const uint64_t steps_g = ((uint64_t)n_cg + rpw - 1) / rpw;
-        const uint64_t grid_cg = std::min<uint64_t>((steps_g + 7) / 8, (uint64_t)sms * CHUNK_MINB);
-        c->begin("bqsr_g_chunk_list", (double)n_cg * (48 + 19 + 8 + 225 + 75));
-        bqsr_chunk_kernel<true><<<(unsigned)grid_cg, 256, smem, c->stream>>>(A, A.cg_list, n_cg);
-        c->end(); LAUNCH_CHECK(c);
-    }
     if (n_gen) {
-        const size_t smem_g = (size_t)c->geom.n_cov * A.n_slots * (2 * Lc + 1 + 16) * 4 * 2;
-        const uint64_t grid_g = std::min<uint64_t>(((uint64_t)n_gen + WARPS_PER_BLOCK - 1) / WARPS_PER_BLOCK, (uint64_t)sms * 4);
-        CUDA_TRY(c, cudaFuncSetAttribute(bqsr_general_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)std::max<size_t>(smem_g, 1024)));
-        c->begin("bqsr_g_warp_per_read", (double)n_gen * (48 + 19 + 225 + 150));
-        bqsr_general_kernel<<<(unsigned)grid_g, WARPS_PER_BLOCK * 32, smem_g, c->stream>>>(A, n_gen);
+        const uint64_t steps_g = ((uint64_t)n_gen + rpw - 1) / rpw;
+        const uint64_t grid_g = std::min<uint64_t>((steps_g + 7) / 8, (uint64_t)sms * CHUNK_MINB);
+        c->begin("bqsr_g_chunk_list", (double)n_gen * (48 + 19 + 8 + 225 + 75));
+        bqsr_chunk_kernel<true><<<(unsigned)grid_g, 256, smem, c->stream>>>(A, A.gen_list, n_gen);
         c->end(); LAUNCH_CHECK(c);
     }
     return E_OK;
@@ -927,9 +774,8 @@ int phase_bqsr_gather(elp_ctx* c) {
         A.n = n; A.refid = c->s_refid.p; A.pos = c->s_pos.p; A.nref = c->s_nref.p; A.pnext = c->s_pnext.p; A.tlen = c->s_tlen.p; A.rg = c->s_rg.p; A.lseq = c->s_lseq.p;
         A.flag = c->s_flag.p; A.mapq = c->s_mapq.p; A.optf = c->s_optf.p; A.qual_off = c->s_qual_off.p; A.seq_off = c->s_seq_off.p; A.cigar_off = c->s_cigar_off.p; A.ncigar = c->s_ncigar.p;
         A.cigar = c->cigar.p; A.seq = c->seq.p; A.qual = c->qual.p; A.rg_cov = c->d_rg_cov; A.n_rg = c->n_rg; A.contig_len = c->d_contig_len; A.n_contigs = c->n_contigs;
-        A.ref = c->d_ref_ptrs; A.ref_len = c->d_ref_len; A.sites = c->d_site_ptrs; A.n_sites = c->d_n_sites;
+        A.refhot = c->d_refhot_ptrs; A.ref_len = c->d_ref_len; A.sites = c->d_site_ptrs; A.n_sites = c->d_n_sites;
         A.geom = c->geom; A.tables = reinterpret_cast<unsigned long long*>(c->d_tables); A.err = c->d_err;
-        A.refnib = c->d_refnib_ptrs;
         uint64_t ref_bytes = 0; for (auto l : c->ref_len) ref_bytes += l;
         // SURVEY.md 8d: N_eligible * (19 + 4 + 4 c + L/2 + L) + genome bytes once; per-read averages of the arenas stand in for c and L
         const double per_read = 23.0 + ((double)c->n_cigar * 4 + (double)(c->n_seq - ARENA_FRONT_PAD) + (double)(c->n_qual - ARENA_FRONT_PAD)) / (double)n;

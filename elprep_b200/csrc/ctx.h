@@ -79,13 +79,9 @@ struct elp_ctx {
     int32_t* d_contig_len = nullptr; // [n_contigs]
 
     // ---- reference genome + known sites (device) ----
-    std::vector<uint8_t*> d_ref;          // per contig
     std::vector<uint64_t> ref_len;
-    const uint8_t** d_ref_ptrs = nullptr; // [n_contigs] device array of pointers
-    std::vector<uint8_t*> d_refnib_raw;   // per contig: 4-bit reference codes (bqsr_gather.cu pack_reference), payload at +32
-    const uint8_t** d_refnib_ptrs = nullptr;
-    std::vector<uint8_t*> d_refhot_raw;   // per contig: one-hot reference nibbles for the count kernel (bqsr_count.inl), payload at +REFHOT_PAD
-    const uint8_t** d_refhot_ptrs = nullptr;
+    std::vector<uint8_t*> d_refhot_raw;   // per contig: one-hot reference nibbles (bqsr_gather.cu pack_reference), payload at +REFHOT_PAD
+    const uint8_t** d_refhot_ptrs = nullptr; // [n_contigs] device array of the payload pointers
     uint64_t* d_ref_len = nullptr;
     std::vector<int32_t*> d_sites;        // per contig, (start,end) pairs
     std::vector<uint64_t> n_sites;
@@ -237,7 +233,7 @@ int phase_bqsr_apply(elp_ctx* c);
 int build_apply_lut(elp_ctx* c, int Lc);   // bqsr_finalize.cu
 int build_compact_lut(elp_ctx* c);
 int upload_side_inputs(elp_ctx* c);
-int pack_reference(elp_ctx* c, int contig);
+int pack_reference(elp_ctx* c, int contig, const uint8_t* bases, uint64_t n);   // bqsr_gather.cu
 int check_device_errors(elp_ctx* c);
 int upload_small(elp_ctx* c, void* dst, const void* src, size_t bytes);   // api.cu: host -> device without the copy engine
 int comm_allreduce_ranges(elp_ctx* c);   // comm.cu
